@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark (BASELINE.json): images/sec @ SDXL 1024^2 50-step & latents/sec @ Flux 1024^2 28-step, 1/2/4/8 B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload all|sdxl|flux|vae|encoders]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload all|sdxl|flux|vae|encoders] [--dump-outputs DIR]
 
 ONE JSON line (rank 0).  Top level = BASELINE config 1: SDXL UNet 1024^2 bf16, batch 1 per GPU (CFG -> 2 samples per
 forward), 50 Euler steps + VAE decode to a (1,3,1024,1024) tensor; a "step" is one whole image.
@@ -23,6 +23,9 @@ With --workload all (default) the line also carries
 --impl reference times the UNMODIFIED reference (baseline/_ref) through its own StableDiffusionXLPipeline on the host cores.
 Multi-GPU: one process per GPU (torchrun), each rank samples its own image (weak scaling), one all-gather of the decoded
 images per step, max-over-ranks device timing.
+Every timed loop runs exactly --steps steps.  --dump-outputs DIR writes what the last timed step of each section returned to
+its caller as DIR/<name>.npy (float32; see Outputs): the inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 import argparse
 import json
@@ -446,6 +449,37 @@ def reference_cuda_eager(unet_cfg, dev, dt):
 
 
 # ----------------------------------------------------------------------------------------------- B200 arm: workloads
+class Outputs:
+    """--dump-outputs: what the last timed step of each section returned, copied to the host as float32 right after its timed
+    loop.  An array of more than `cap` elements is replaced by a fixed sample of its flattened values (indices drawn by
+    torch.randint from seed 0, sorted): the SDXL images get 2^22 elements, every other array 2^20, so that the whole dump
+    (at most 12 arrays) stays under 64 MB."""
+    FLAGSHIP_CAP, CAP = 1 << 22, 1 << 20
+
+    def __init__(self, directory):
+        self.dir, self.arrays = directory, {}
+
+    def keep(self, name, t, cap=CAP):
+        if self.dir is None:
+            return
+        t = t.detach()
+        if t.numel() > cap:
+            idx = torch.randint(t.numel(), (cap,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        self.arrays[name] = t.float().cpu().numpy()
+
+    def write(self):
+        if self.dir is None:
+            return
+        import numpy as np
+        os.makedirs(self.dir, exist_ok=True)
+        assert sum(a.nbytes for a in self.arrays.values()) <= 64 << 20
+        for name, a in self.arrays.items():
+            np.save(os.path.join(self.dir, name + ".npy"), a)
+
+
+OUTPUTS = Outputs(None)  # main() sets the directory on rank 0
+
 class Ctx:
     def __init__(self, args, rank, world, local_rank):
         self.args, self.rank, self.world, self.local_rank = args, rank, world, local_rank
@@ -455,6 +489,7 @@ class Ctx:
         self.pk = peaks()
         self.gpu_dead = False
         self.flux_state = None
+        self.last = None  # what body() returned in the last step of the last timed loop
 
     def barrier(self):
         if self.world > 1:
@@ -470,7 +505,7 @@ class Ctx:
         n0 = ops.launches()
         e0.record()
         for i in range(n):
-            body(i)
+            self.last = body(i)
         e1.record()
         self.barrier()
         ms = e0.elapsed_time(e1)
@@ -516,6 +551,8 @@ def sdxl_section(cx):
         one_image(resident, i, False)
     with ClockSampler(cx.local_rank) as cs:
         ms, launches = cx.timed(args.steps, lambda i: one_image(resident, 1000 + i, False))
+    OUTPUTS.keep("sdxl_images", cx.last, Outputs.FLAGSHIP_CAP)
+    cx.last = None
     clocks = cs.summary()
     h2d = lambda: {k: v.to(dev, non_blocking=True) for k, v in host.items()}  # noqa: E731
     one_image(h2d(), 0, True)
@@ -572,9 +609,11 @@ def config3_section(cx, pipe):
         return to_host(imgs) if cx.rank == 0 else imgs
 
     batch(0)
-    n = max(1, min(args.steps, 2))
+    n = args.steps
     with ClockSampler(cx.local_rank) as cs:
         ms, launches = cx.timed(n, lambda i: batch(10 + i))
+    OUTPUTS.keep("config3_images", cx.last)
+    cx.last = None
     return dict(workload=f"sdxl_1024_{args.denoise_steps}step_cfg{args.guidance_scale}_global_batch{Bg}_b4_per_gpu(B_eff 8)",
                 value=round(n * Bg / (ms * 1e-3), 4), unit="images/s", ms_per_batch=round(ms / n, 1), batches_timed=n, e2e=True,
                 h2d_bytes_per_step=sum(v.numel() * v.element_size() for v in host.values()), d2h_bytes_per_step=Bg * 3 * 1024 * 1024 * 2,
@@ -582,7 +621,7 @@ def config3_section(cx, pipe):
                 note="one seeded full-batch latent draw sliced per rank (parallel.sdxl_data_parallel); host embeddings in, all images to rank 0's host")
 
 
-def flux_section(cx, standalone=False):
+def flux_section(cx):
     """BASELINE configs[2]: latents/sec, FluxTransformer2DModel (Flux.1-dev shape), 1024^2 (4096 image + 512 text tokens),
     28 FlowMatch steps, guidance 3.5, output_type='latent'.  N > 1: one latent per GPU per step (replicas, weak scaling)."""
     from diffusers_b200.pipelines import FluxPipeline
@@ -603,7 +642,7 @@ def flux_section(cx, standalone=False):
                 pooled_prompt_embeds=torch.randn(1, 768, generator=g).to(dt).pin_memory())
     nsteps = 28 if args.denoise_steps == 50 else args.denoise_steps
     call = dict(height=1024, width=1024, num_inference_steps=nsteps, guidance_scale=3.5, output_type="latent")
-    n = max(args.steps, 5) if not standalone else args.steps
+    n = args.steps
 
     def one(emb, seed, host_out):
         lat = pipe(generator=torch.Generator(device=dev).manual_seed(seed), **emb, **call).images
@@ -614,6 +653,8 @@ def flux_section(cx, standalone=False):
         one(res, i, False)
     with ClockSampler(cx.local_rank) as cs:
         ms, launches = cx.timed(n, lambda i: one(res, 100 + i, False))
+    OUTPUTS.keep("flux_latents", cx.last)
+    cx.last = None
     ms2, _ = cx.timed(n, lambda i: one({k: v.to(dev, non_blocking=True) for k, v in host.items()}, 200 + i, True))
     value = n * world / (ms * 1e-3)
     fl = nsteps * FLUX_FLOP_PER_FORWARD
@@ -661,9 +702,11 @@ def flux_context_parallel(cx, pipe, tr, res, call, nsteps, replica_ms):
             return pipe(generator=torch.Generator(device=dev).manual_seed(seed), **res, **call).images
 
         one(0)
-        n = max(2, min(args.steps, 3))
+        n = args.steps
         with ClockSampler(cx.local_rank) as cs:
             ms, launches = cx.timed(n, lambda i: one(300 + i))
+        OUTPUTS.keep("flux_context_parallel_latents", cx.last)
+        cx.last = None
         _, bufs = next(iter(tr._cp["plans"].values()))
         return dict(ulysses_degree=world, scaling="strong", value=round(n / (ms * 1e-3), 4), unit="latents/s", ms_per_latent=round(ms / n, 1),
                     ms_per_forward=round(ms / n / nsteps, 2), one_gpu_ms_per_latent=round(replica_ms, 1), speedup_vs_one_gpu=round(replica_ms / (ms / n), 3),
@@ -689,8 +732,10 @@ def vae_section(cx):
             z = zh.to(dev)
             for _ in range(max(1, args.warmup if B < 64 else 1)):
                 vae.decode(z, return_dict=False)
-            n = max(1, args.steps if B < 64 else min(args.steps, 2))
+            n = args.steps
             ms, launches = cx.timed(n, lambda i: vae.decode(z, return_dict=False))
+            OUTPUTS.keep(f"vae_decode_b{B}", cx.last[0])
+            cx.last = None
             ms2, _ = cx.timed(n, lambda i: to_host(vae.decode(zh.to(dev, non_blocking=True), return_dict=False)[0]))
             sweep[B] = dict(images_per_s=round(B * n / (ms * 1e-3), 2), ms_per_batch=round(ms / n, 2), e2e_images_per_s=round(B * n / (ms2 * 1e-3), 2),
                             tflops=round(B * n * VAE_FLOP_PER_IMAGE / (ms * 1e-3) / 1e12, 1), launches=launches // n)
@@ -733,7 +778,7 @@ def encoders_section(cx):
     te2 = mk(T.CLIPTextModelWithProjection, T.CLIP_BIGG_CONFIG, T.clip_text_params(T.CLIP_BIGG_CONFIG, True), 2)
     g = torch.Generator().manual_seed(3)
     ids77 = torch.randint(3, 49000, (2, 77), generator=g).pin_memory()  # prompt + negative prompt
-    n = max(3, args.steps)
+    n = args.steps
 
     def sdxl_encode(i):
         ids = ids77.to(dev, non_blocking=True)
@@ -742,6 +787,8 @@ def encoders_section(cx):
 
     sdxl_encode(0)
     ms, launches = cx.timed(n, sdxl_encode)
+    OUTPUTS.keep("sdxl_text_encode_hidden_states", cx.last[0])
+    OUTPUTS.keep("sdxl_text_encode_pooled", cx.last[1])
     out["sdxl_text_encode"] = dict(value=round(n / (ms * 1e-3), 2), unit="prompt pairs/s", ms=round(ms / n, 3), gpu_launches=launches // n,
                                    models="CLIPTextModel (CLIP-L, 123 M) + CLIPTextModelWithProjection (OpenCLIP bigG, 695 M), 2 x 77 tokens",
                                    h2d_bytes_per_step=ids77.numel() * 8, d2h_bytes_per_step=2 * 77 * 2048 * 2 + 2 * 1280 * 2)
@@ -756,6 +803,8 @@ def encoders_section(cx):
 
     flux_encode(0)
     ms, launches = cx.timed(n, flux_encode)
+    OUTPUTS.keep("flux_text_encode_prompt_embeds", cx.last[0])
+    OUTPUTS.keep("flux_text_encode_pooled", cx.last[1])
     out["flux_text_encode"] = dict(value=round(n / (ms * 1e-3), 2), unit="prompts/s", ms=round(ms / n, 3), gpu_launches=launches // n,
                                    models="CLIPTextModel (CLIP-L) on 77 tokens + T5EncoderModel (T5-XXL v1.1, 4.76 B) on 512 tokens",
                                    h2d_bytes_per_step=(77 + 512) * 8, d2h_bytes_per_step=512 * 4096 * 2 + 768 * 2)
@@ -769,6 +818,8 @@ def encoders_section(cx):
 
     enc(0)
     ms, launches = cx.timed(n, enc)
+    OUTPUTS.keep("vae_encode_moments", cx.last)
+    cx.last = None
     out["vae_encode"] = dict(value=round(n / (ms * 1e-3), 2), unit="images/s", ms=round(ms / n, 3), gpu_launches=launches // n,
                              workload="AutoencoderKL.encode 1024^2 -> moments (SDXL VAE encoder, 34 M params)", h2d_bytes_per_step=3 * 1024 * 1024 * 2,
                              d2h_bytes_per_step=8 * 128 * 128 * 2)
@@ -781,7 +832,7 @@ def run_b200(args, rank, world, local_rank):
     cx = Ctx(args, rank, world, local_rank)
     wl = args.workload
     if wl == "flux":
-        line = flux_section(cx, standalone=True)
+        line = flux_section(cx)
     elif wl == "vae":
         line = vae_section(cx) if rank == 0 else None
     elif wl == "encoders":
@@ -810,18 +861,24 @@ def run_b200(args, rank, world, local_rank):
     if cx.flux_state is not None:
         # ONE latent over all N GPUs (context parallelism over peer memory).  It is the only section in which a rank can wait for a
         # peer inside a kernel, so it runs last and under a watchdog: whatever happens to it, rank 0 prints the line it already has.
+        # The limit covers the set-up, the warm-up latent and 10 s per timed latent (one took 1.2 s on 2 B200s, profiles/README.md).
         import threading
+        limit = 240.0 + 10.0 * args.steps
         sec = line if wl == "flux" else line["flux"]
-        sec["context_parallel"] = "failed: no result within 240 s (watchdog)"
+        sec["context_parallel"] = f"failed: no result within {limit:.0f} s (watchdog)"
 
         def give_up():
             if rank == 0:
                 emit(line)
+                try:
+                    OUTPUTS.write()
+                except Exception as e:  # noqa: BLE001  (the process ends here either way)
+                    sys.stderr.write(f"--dump-outputs failed: {type(e).__name__}: {e}\n")
             sys.stdout.flush()
             sys.stderr.flush()
             os._exit(0)
 
-        dog = threading.Timer(240.0, give_up)
+        dog = threading.Timer(limit, give_up)
         dog.daemon = True
         dog.start()
         res = flux_context_parallel(cx, *cx.flux_state)
@@ -830,6 +887,7 @@ def run_b200(args, rank, world, local_rank):
         cx.flux_state = None
     if rank == 0 and line is not None:
         emit(line)
+        OUTPUTS.write()  # after the line: a failed dump must not cost it
     if cx.gpu_dead:  # a trapped kernel left the CUDA context unusable: the line is out, skip the collective teardown
         sys.stdout.flush()
         sys.stderr.flush()
@@ -870,8 +928,13 @@ def main():
     ap.add_argument("--no-context-parallel", action="store_true", help="N > 1: skip the Flux context-parallel (one latent over N GPUs) measurement")
     ap.add_argument("--no-reference-cuda", action="store_true")
     ap.add_argument("--cpu-sample", action="store_true", help="with --impl reference: print only the bounded cpu_baseline sample (used by the B200 arm)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step of each section to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
+    if rank == 0:
+        OUTPUTS.dir = args.dump_outputs
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":

@@ -8,6 +8,8 @@ the committed files only hold configs, seeds, inputs and the reference's outputs
 store the (tiny) reference-initialised state_dicts, because the reference's hard-coded golden slices
 (tests/models/unets/test_unet_2d_blocks.py) are defined for the reference's own seeded default init.
 """
+import gzip
+import json
 import os
 import sys
 
@@ -548,11 +550,149 @@ def gen_text(d):
     torch.save(out, os.path.join(OUT, "text.pt"))
 
 
+def _inventory(sd):
+    return {k: tuple(v.shape) for k, v in sd.items()}
+
+
+def _files(root):
+    """Every file under root: JSON files by content, safetensors files by metadata and {key: (dtype, shape)}."""
+    from safetensors import safe_open
+    out = {}
+    for dp, _, fs in os.walk(root):
+        for f in sorted(fs):
+            p = os.path.join(dp, f)
+            rel = os.path.relpath(p, root)
+            if f.endswith(".json"):
+                with open(p) as fh:
+                    out[rel] = json.load(fh)
+            elif f.endswith(".safetensors"):
+                with safe_open(p, "pt") as st:
+                    out[rel] = dict(metadata=st.metadata(), tensors={k: (str(st.get_tensor(k).dtype), tuple(st.get_tensor(k).shape)) for k in st.keys()})
+            else:
+                out[rel] = None
+    return out
+
+
+def gen_reference_api(d):
+    """tests/golden/reference_api.json.gz: what the CPU tests of the reference-facing API (parameter inventories, checkpoint files,
+    guidance_rescale) compared with the live reference, recorded so that they run without it.
+      inventories      : state_dict names -> shapes of the reference modules (meta device) at the BASELINE.json sizes
+      loaded           : for each micro model of tests/test_checkpoint.py, the reference's `from_pretrained` of what the shell's
+                         `save_pretrained` wrote: loading info and state_dict names -> shapes
+      save_pretrained  : the files the reference writes for a micro UNet2DModel (sharded, fp16 variant, DDPMPipeline): JSON
+                         contents verbatim, safetensors files as metadata + names / dtypes / shapes
+      rescale_noise_cfg: the reference function's outputs on seeded bf16 inputs (exact in JSON: bf16 values are doubles)"""
+    import tempfile
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import test_checkpoint as tc
+    from diffusers_b200.autoencoder_kl import AutoencoderKL
+    out = {}
+    with torch.device("meta"):
+        out["inventories"] = dict(
+            sdxl_unet=_inventory(d.UNet2DConditionModel(**specs.SDXL_UNET_CONFIG).state_dict()),
+            sdxl_vae=_inventory(d.AutoencoderKL(**specs.SDXL_VAE_CONFIG).state_dict()),
+            flux_dev=_inventory(d.FluxTransformer2DModel(**specs.FLUX_DEV_CONFIG).state_dict()),
+            ddpm_tiny=_inventory(d.UNet2DModel(**specs.DDPM_TINY_CONFIG).state_dict()))
+    loaded = {}
+    cases = [(n, cls, dflt, micro, fn) for n, cls, dflt, micro, fn in tc.CASES if n != "AutoencoderKL"]
+    cases.append(("AutoencoderKL", AutoencoderKL, specs.SDXL_VAE_CONFIG, tc.MICRO_VAE, specs.vae_params))
+    with tempfile.TemporaryDirectory() as tmp:
+        for name, cls, defaults, micro, spec_fn in cases:
+            cfg = dict(defaults)
+            cfg.update(micro)
+            sd = specs.random_state_dict(spec_fn(cfg), seed=11, dtype=torch.bfloat16)
+            exact = dict(fold_norms=False) if name == "UNet2DConditionModel" else {}
+            cls(cfg, sd, device="cpu", **exact).save_pretrained(os.path.join(tmp, name))
+            ref, info = getattr(d, name).from_pretrained(os.path.join(tmp, name), torch_dtype=torch.bfloat16, output_loading_info=True)
+            loaded[name] = dict(cfg=cfg, info={k: list(v) for k, v in info.items()}, state_dict=_inventory(ref.state_dict()))
+            print("loaded", name, len(loaded[name]["state_dict"]), {k: len(v) for k, v in info.items()})
+    out["loaded"] = loaded
+    cfg = dict(specs.DDPM_TINY_CONFIG)
+    cfg.update(tc.MICRO_DDPM)
+    torch.manual_seed(0)
+    m = d.UNet2DModel(**cfg).to(torch.bfloat16)
+    with tempfile.TemporaryDirectory() as tmp:
+        m.save_pretrained(os.path.join(tmp, "u"), safe_serialization=True, max_shard_size="300KB")
+        m.save_pretrained(os.path.join(tmp, "v"), safe_serialization=True, variant="fp16")
+        d.DDPMPipeline(unet=m, scheduler=d.DDPMScheduler()).save_pretrained(os.path.join(tmp, "p"))
+        out["save_pretrained"] = dict(cfg=cfg, dirs={k: _files(os.path.join(tmp, k)) for k in ("u", "v", "p")})
+    from diffusers.pipelines.stable_diffusion_xl.pipeline_stable_diffusion_xl import rescale_noise_cfg
+    g = torch.Generator().manual_seed(0)
+    cfg_pred, text_pred = torch.randn(3, 4, 8, 8, generator=g).bfloat16() * 2, torch.randn(3, 4, 8, 8, generator=g).bfloat16()
+    out["rescale_noise_cfg"] = {str(gr): rescale_noise_cfg(cfg_pred, text_pred, guidance_rescale=gr).float().tolist() for gr in (0.0, 0.3, 0.7, 1.0)}
+    with gzip.GzipFile(os.path.join(OUT, "reference_api.json.gz"), "wb", mtime=0) as f:
+        f.write(json.dumps(out).encode())
+
+
+def gen_full_size(d):
+    """tests/golden/full_size_reference.pt (needs a B200): the reference at the full sizes of tests/test_full_size_parity_gpu.py,
+    on that test's weights and seeded CUDA inputs.  Per case: the test's fixed _sample() of the fp32 output, its shape, and the
+    error of the reference's own 16-bit CUDA-eager run (the same calls as that test's live branch) against that fp32 output:
+    ref16_mean_abs, ref16_max_abs, ref16_in_band_vs_fp32, the yardstick of the test's criterion."""
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import test_full_size_parity_gpu as fs
+    fs._no_tf32()
+    dev = fs.DEV
+    out = {}
+
+    def keep(name, r32, r16):
+        e16 = (r16.float() - r32).abs()
+        out[name] = dict(sample=fs._sample(r32), shape=tuple(r32.shape), ref16_mean_abs=float(e16.mean()), ref16_max_abs=float(e16.max()),
+                         ref16_in_band_vs_fp32=fs._band(r16.float(), r32))
+        print(name, {k: v for k, v in out[name].items() if k != "sample"}, float(r32.abs().max()))
+
+    with torch.no_grad():
+        cfg = dict(specs.SDXL_UNET_CONFIG)
+        t = torch.tensor(981.0, device=dev)
+        for dt, tag in ((torch.bfloat16, "bf16"), (torch.float16, "fp16")):
+            sd32 = {k: v.float() for k, v in specs.random_state_dict(specs.unet2d_condition_params(cfg), seed=0, dtype=dt, device=dev).items()}
+            x, ehs, te, tid = fs._sdxl_inputs(dt)
+            m = fs._ref_module("UNet2DConditionModel", cfg, sd32, torch.float32)
+            r32 = m(x.float(), t, ehs.float(), added_cond_kwargs=dict(text_embeds=te.float(), time_ids=tid.float()), return_dict=False)[0]
+            m = m.to(dt)
+            keep(f"sdxl_unet_{tag}", r32, m(x, t, ehs, added_cond_kwargs=dict(text_embeds=te, time_ids=tid), return_dict=False)[0])
+            del m, sd32, r32
+            fs._free()
+        dt = torch.bfloat16
+        cfg = dict(specs.SDXL_VAE_CONFIG)
+        sd32 = {k: v.float() for k, v in specs.random_state_dict(specs.vae_decoder_params(cfg), seed=0, dtype=dt, device=dev).items()}
+        z = fs._vae_decode_inputs(dt)
+        m = fs._ref_module("AutoencoderKL", cfg, sd32, torch.float32, strict=False)
+        r32 = m.decode(z.float(), return_dict=False)[0]
+        m.decoder.to(dt)
+        m.post_quant_conv.to(dt)
+        keep("sdxl_vae_decode", r32, m.decode(z, return_dict=False)[0])
+        del m, sd32
+        sd32 = {k: v.float() for k, v in specs.random_state_dict(specs.vae_params(cfg), seed=0, dtype=dt, device=dev).items()}
+        x = fs._vae_encode_inputs(dt)
+        m = fs._ref_module("AutoencoderKL", cfg, sd32, torch.float32)
+        r32 = m.encode(x.float()).latent_dist.parameters
+        m = m.to(dt)
+        keep("sdxl_vae_encode", r32, m.encode(x).latent_dist.parameters)
+        del m, sd32
+        fs._free()
+        cfg = dict(specs.FLUX_DEV_CONFIG)
+        sd16 = specs.random_state_dict(specs.flux_params(cfg), seed=0, dtype=dt, device=dev)
+        hs, ehs, pooled, img_ids, txt_ids, ts, guidance = fs._flux_inputs(dt)
+        m = fs._ref_module("FluxTransformer2DModel", cfg, sd16, dt)
+        r16 = m(hidden_states=hs, encoder_hidden_states=ehs, pooled_projections=pooled, timestep=ts, img_ids=img_ids, txt_ids=txt_ids,
+                guidance=guidance, return_dict=False)[0]
+        del m
+        sd32 = {k: v.float() for k, v in sd16.items()}
+        del sd16
+        fs._free()
+        m = fs._ref_module("FluxTransformer2DModel", cfg, sd32, torch.float32)
+        keep("flux_dev_shape", m(hidden_states=hs.float(), encoder_hidden_states=ehs.float(), pooled_projections=pooled.float(), timestep=ts.float(),
+                                 img_ids=img_ids.float(), txt_ids=txt_ids.float(), guidance=guidance, return_dict=False)[0], r16)
+    torch.save(out, os.path.join(OUT, "full_size_reference.pt"))
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
     torch.set_num_threads(8)
     dmod = ref_shim.import_reference()
-    which = sys.argv[1:] or ["blocks", "layers", "schedulers", "steppers", "models", "pipelines", "checkpoints", "vae_encode", "text"]
+    which = sys.argv[1:] or ["blocks", "layers", "schedulers", "steppers", "models", "pipelines", "checkpoints", "vae_encode", "text",
+                             "reference_api"]
     for w in which:
         globals()["gen_" + w](dmod)
     for f in sorted(os.listdir(OUT)):

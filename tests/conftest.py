@@ -39,6 +39,16 @@ def golden():
     return load
 
 
+@pytest.fixture(scope="session")
+def reference_api():
+    """What the reference's own API returned for the tests that pin parameter inventories, checkpoint files and helper
+    functions against it (oracle/make_golden.py, gen_reference_api)."""
+    import gzip
+    import json
+    with gzip.open(os.path.join(GOLDEN, "reference_api.json.gz"), "rt") as f:
+        return json.load(f)
+
+
 def state_dicts(spec, seed):
     """(bf16, fp32-upcast) weights exactly as oracle/make_golden.py generated them."""
     import torch

@@ -192,22 +192,37 @@ def test_reference_written_pipeline_directory():
         DDPMPipeline.from_pretrained(FIXTURE, device="cpu")
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="needs the reference (build container only)")
-def test_reference_save_pretrained_round_trip(tmp_path):
-    """The real writer, today: reference model -> save_pretrained -> shell.from_pretrained == shell(state_dict)."""
-    from oracle import ref_shim
-    d = ref_shim.import_reference()
+def _write_recorded(root, files, sd):
+    """Re-creates a directory the reference's save_pretrained wrote (tests/golden/reference_api.json.gz): its JSON files
+    verbatim, each safetensors file with the recorded metadata and the recorded tensor names / dtypes / shapes, valued from sd."""
+    from safetensors.torch import save_file
+    for rel, content in files.items():
+        p = os.path.join(root, rel)
+        os.makedirs(os.path.dirname(p), exist_ok=True)
+        if rel.endswith(".json"):
+            with open(p, "w") as f:
+                json.dump(content, f)
+        else:
+            tensors = {}
+            for k, (dtype, shape) in content["tensors"].items():
+                assert str(sd[k].dtype) == dtype and tuple(sd[k].shape) == tuple(shape), k
+                tensors[k] = sd[k].contiguous()
+            save_file(tensors, p, metadata=content["metadata"])
+
+
+def test_reference_save_pretrained_round_trip(tmp_path, reference_api):
+    """The real writer: reference model -> save_pretrained -> shell.from_pretrained == shell(state_dict)."""
+    rec = reference_api["save_pretrained"]
     cfg = dict(specs.DDPM_TINY_CONFIG)
     cfg.update(MICRO_DDPM)
-    torch.manual_seed(0)
-    m = d.UNet2DModel(**cfg).to(torch.bfloat16)
-    m.save_pretrained(str(tmp_path / "u"), safe_serialization=True, max_shard_size="300KB")  # forces the sharded layout
-    assert os.path.isfile(tmp_path / "u" / "diffusion_pytorch_model.safetensors.index.json")
+    assert json.loads(json.dumps(cfg)) == rec["cfg"]
+    sd = specs.random_state_dict(specs.unet2d_params(cfg), seed=0, dtype=torch.bfloat16)
+    for k in ("u", "v", "p"):
+        _write_recorded(str(tmp_path / k), rec["dirs"][k], sd)
+    assert os.path.isfile(tmp_path / "u" / "diffusion_pytorch_model.safetensors.index.json")  # max_shard_size="300KB": sharded layout
     ours = UNet2DModel.from_pretrained(str(tmp_path / "u"), device="cpu")
-    _same_buffers(UNet2DModel(cfg, {k: v for k, v in m.state_dict().items()}, device="cpu"), ours)
-    m.save_pretrained(str(tmp_path / "v"), safe_serialization=True, variant="fp16")
+    _same_buffers(UNet2DModel(cfg, sd, device="cpu"), ours)
     _same_buffers(ours, UNet2DModel.from_pretrained(str(tmp_path / "v"), variant="fp16", device="cpu"))
-    d.DDPMPipeline(unet=m, scheduler=d.DDPMScheduler()).save_pretrained(str(tmp_path / "p"))
     p = DDPMPipeline.from_pretrained(str(tmp_path / "p"), device="cpu")
     _same_buffers(ours, p.unet)
     assert isinstance(p.scheduler, DDPMScheduler) and p.scheduler.config.num_train_timesteps == 1000
@@ -255,23 +270,29 @@ def test_unet_conv_projection_and_multi_layer_round_trip():
             assert back["mid_block.attentions.0.proj_in.weight"].dim() == 4
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="needs the reference (build container only)")
-def test_unmodified_reference_loads_what_the_shells_save(tmp_path):
+def _reference_loads(path, rec, sd):
+    """What the reference's from_pretrained (recorded in tests/golden/reference_api.json.gz) reports for the same model: no
+    missing / unexpected / mismatched keys, and its state_dict names and shapes are exactly those of the saved file, which
+    holds sd's values."""
+    assert not any(rec["info"].values()), rec["info"]
+    saved = checkpoint.load_state_dict(path)
+    assert {k: tuple(v.shape) for k, v in saved.items()} == {k: tuple(s) for k, s in rec["state_dict"].items()}
+    assert all(torch.equal(saved[k], sd[k]) for k in sd)
+
+
+def test_unmodified_reference_loads_what_the_shells_save(tmp_path, reference_api):
     """shell.save_pretrained -> the reference's own from_pretrained: same parameters, no missing / unexpected keys."""
-    from oracle import ref_shim
-    d = ref_shim.import_reference()
     for name, cls, defaults, micro, spec_fn in CASES:
         if name == "AutoencoderKL":
             continue
         cfg = dict(defaults)
         cfg.update(micro)
+        rec = reference_api["loaded"][name]
+        assert json.loads(json.dumps(cfg)) == rec["cfg"]
         sd = specs.random_state_dict(spec_fn(cfg), seed=11, dtype=torch.bfloat16)
         exact = dict(fold_norms=False) if name == "UNet2DConditionModel" else {}
         cls(cfg, sd, device="cpu", **exact).save_pretrained(str(tmp_path / name))
-        ref, info = getattr(d, name).from_pretrained(str(tmp_path / name), torch_dtype=torch.bfloat16, output_loading_info=True)
-        assert not info["missing_keys"] and not info["unexpected_keys"] and not info["mismatched_keys"], info
-        rsd = ref.state_dict()
-        assert all(torch.equal(rsd[k], sd[k]) for k in sd)
+        _reference_loads(str(tmp_path / name), rec, sd)
 
 
 @pytest.mark.parametrize("kind", ["clip", "clip_proj", "t5"])
@@ -311,7 +332,7 @@ def test_text_encoder_shells_load_transformers_checkpoints(tmp_path, kind):
         (T.T5EncoderModel if kind != "t5" else T.CLIPTextModel).from_pretrained(str(tmp_path), subfolder="text_encoder", device="cpu")
 
 
-def test_whole_vae_checkpoint_round_trip(tmp_path):
+def test_whole_vae_checkpoint_round_trip(tmp_path, reference_api):
     """With the encoder half loaded (N3) the AutoencoderKL shell holds the reference's complete state_dict: reference_state_dict()
     is the exact inverse of the packing for encoder.* / quant_conv.* too, save_pretrained writes a directory that from_pretrained
     reads back WITH the encoder - and that the unmodified reference loads without missing / unexpected keys."""
@@ -332,10 +353,4 @@ def test_whole_vae_checkpoint_round_trip(tmp_path):
     # a checkpoint that lacks part of the encoder is an error, not a silent decoder-only model
     with pytest.raises(ValueError):
         AutoencoderKL(cfg, {k: v for k, v in sd.items() if k != "encoder.conv_out.bias"}, device="cpu")
-    if os.path.isdir("/root/reference/src"):
-        from oracle import ref_shim
-        d = ref_shim.import_reference()
-        ref, info = d.AutoencoderKL.from_pretrained(str(tmp_path / "vae"), torch_dtype=torch.bfloat16, output_loading_info=True)
-        assert not info["missing_keys"] and not info["unexpected_keys"] and not info["mismatched_keys"], info
-        rsd = ref.state_dict()
-        assert all(torch.equal(rsd[k], sd[k]) for k in sd)
+    _reference_loads(str(tmp_path / "vae"), reference_api["loaded"]["AutoencoderKL"], sd)

@@ -171,7 +171,7 @@ def _run_two(worker):
 
 
 def _peer_failure_worker(rank, world, port, q_out):
-    """No GPU here, so b200_peer_alloc fails on every rank: the failure must surface as the SAME error on all ranks (after the outcome
+    """b200_peer_alloc fails on every rank: the failure must surface as the SAME error on all ranks (after the outcome
     exchange), not as one rank raising while the other waits in a collective."""
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
@@ -180,8 +180,23 @@ def _peer_failure_worker(rank, world, port, q_out):
         import torch.cuda
         from diffusers_b200 import _lib
         from diffusers_b200 import context_parallel as cp
+        real = _lib.lib()
+
+        class NoPeerMemory:  # the allocation fails as it does without a device, whether or not this host has a GPU
+            def __getattr__(self, name):
+                return getattr(real, name)
+
+            @staticmethod
+            def b200_peer_alloc(nbytes, ptr, handle):
+                return 1
+
+            @staticmethod
+            def b200_last_error():
+                return b"no CUDA device"
+
         torch.cuda.current_device = lambda: 0      # host-only stand-ins: the allocation itself is what must fail
         _lib.init = lambda d: None
+        _lib.lib = lambda: NoPeerMemory()
         try:
             cp.PeerBuffer(1 << 20)
             q_out.put((rank, "no error"))

@@ -67,19 +67,14 @@ def test_specs_full_size_parameter_counts():
     assert n(specs.vae_decoder_params(specs.SDXL_VAE_CONFIG)) == 49_490_199  # decoder 49.49 M + post_quant_conv
 
 
-def test_specs_match_reference_state_dicts():
-    from oracle import ref_shim
-    if not ref_shim.available():
-        pytest.skip("reference not present on this box")
-    d = ref_shim.import_reference()
-    with torch.device("meta"):
-        pairs = [(d.UNet2DConditionModel(**specs.SDXL_UNET_CONFIG).state_dict(), specs.unet2d_condition_params(specs.SDXL_UNET_CONFIG)),
-                 (d.FluxTransformer2DModel(**specs.FLUX_DEV_CONFIG).state_dict(), specs.flux_params(specs.FLUX_DEV_CONFIG)),
-                 (d.UNet2DModel(**specs.DDPM_TINY_CONFIG).state_dict(), specs.unet2d_params(specs.DDPM_TINY_CONFIG))]
-        v = d.AutoencoderKL(**specs.SDXL_VAE_CONFIG).state_dict()
-        pairs.append(({k: t for k, t in v.items() if k.startswith(("decoder", "post_quant"))}, specs.vae_decoder_params(specs.SDXL_VAE_CONFIG)))
+def test_specs_match_reference_state_dicts(reference_api):
+    inv = reference_api["inventories"]  # the reference modules' state_dict shapes on the meta device
+    pairs = [(inv["sdxl_unet"], specs.unet2d_condition_params(specs.SDXL_UNET_CONFIG)),
+             (inv["flux_dev"], specs.flux_params(specs.FLUX_DEV_CONFIG)),
+             (inv["ddpm_tiny"], specs.unet2d_params(specs.DDPM_TINY_CONFIG)),
+             ({k: s for k, s in inv["sdxl_vae"].items() if k.startswith(("decoder", "post_quant"))}, specs.vae_decoder_params(specs.SDXL_VAE_CONFIG))]
     for ref, mine in pairs:
-        assert {k: tuple(t.shape) for k, t in ref.items()} == {k: tuple(s) for k, s in mine.items()}
+        assert {k: tuple(s) for k, s in ref.items()} == {k: tuple(s) for k, s in mine.items()}
 
 
 def test_randn_tensor_contract():
@@ -239,18 +234,15 @@ def test_unet_fold_norms_flag_keeps_exact_weights_when_off():
         assert d <= tol, (k, float(d))
 
 
-def test_rescale_noise_cfg_is_the_references(monkeypatch):
+def test_rescale_noise_cfg_is_the_references(monkeypatch, reference_api):
     """N4: guidance_rescale.  The formula against the unmodified reference's function on the same 16-bit tensors (bit for bit), and
     the SDXL drop-in loop applying it after the CFG combine (fake denoiser / stepper: the loop is glue, the kernels are tested elsewhere)."""
-    from baseline import ref_env
     from diffusers_b200.pipelines import StableDiffusionXLPipeline, rescale_noise_cfg
     g = torch.Generator().manual_seed(0)
     cfg_pred, text_pred = torch.randn(3, 4, 8, 8, generator=g).bfloat16() * 2, torch.randn(3, 4, 8, 8, generator=g).bfloat16()
-    if ref_env.available():
-        ref_env.import_reference()
-        from diffusers.pipelines.stable_diffusion_xl.pipeline_stable_diffusion_xl import rescale_noise_cfg as ref_fn
-        for gr in (0.0, 0.3, 0.7, 1.0):
-            assert torch.equal(rescale_noise_cfg(cfg_pred, text_pred, gr), ref_fn(cfg_pred, text_pred, guidance_rescale=gr)), gr
+    for gr in (0.0, 0.3, 0.7, 1.0):
+        ref = torch.tensor(reference_api["rescale_noise_cfg"][str(gr)]).bfloat16()  # the reference's output, recorded
+        assert torch.equal(rescale_noise_cfg(cfg_pred, text_pred, gr), ref), gr
     out = rescale_noise_cfg(cfg_pred.float(), text_pred.float(), 1.0)
     assert torch.allclose(out.std(dim=[1, 2, 3]), text_pred.float().std(dim=[1, 2, 3]), rtol=1e-5)  # full rescale: the text prediction's std per sample
 

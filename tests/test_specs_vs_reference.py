@@ -1,22 +1,14 @@
 """diffusers_b200.specs restates the reference constructors' parameter inventory; this checks every name and shape against
-the UNMODIFIED reference's own modules built on the meta device (no memory, no arithmetic), at the BASELINE.json sizes.
-Runs wherever the reference is importable (baseline/_ref travels to the GPU box; /root/reference in the build container)."""
+the UNMODIFIED reference's own modules built on the meta device, at the BASELINE.json sizes, as recorded by
+oracle/make_golden.py (gen_reference_api) in tests/golden/reference_api.json.gz."""
 import pytest
 import torch
 
-from baseline import ref_env
 from diffusers_b200 import specs
 
-pytestmark = pytest.mark.skipif(not ref_env.available(), reason="reference not installed (baseline/_ref) and /root/reference absent")
 
-
-def _meta(cls, cfg):
-    with torch.device("meta"):
-        return cls(**cfg)
-
-
-def _compare(spec, module, prefix_filter=None):
-    ref = {k: tuple(v.shape) for k, v in module.state_dict().items() if prefix_filter is None or prefix_filter(k)}
+def _compare(spec, inventory, prefix_filter=None):
+    ref = {k: tuple(v) for k, v in inventory.items() if prefix_filter is None or prefix_filter(k)}
     ours = {k: tuple(v) for k, v in spec.items()}
     assert sorted(ours) == sorted(ref), (sorted(set(ours) - set(ref))[:5], sorted(set(ref) - set(ours))[:5])
     bad = [(k, ours[k], ref[k]) for k in ours if ours[k] != ref[k]]
@@ -24,32 +16,27 @@ def _compare(spec, module, prefix_filter=None):
     return len(ours)
 
 
-def test_sdxl_unet_names_and_shapes():
-    d = ref_env.import_reference()
-    n = _compare(specs.unet2d_condition_params(specs.SDXL_UNET_CONFIG), _meta(d.UNet2DConditionModel, specs.SDXL_UNET_CONFIG))
+def test_sdxl_unet_names_and_shapes(reference_api):
+    n = _compare(specs.unet2d_condition_params(specs.SDXL_UNET_CONFIG), reference_api["inventories"]["sdxl_unet"])
     assert n == 1680  # stabilityai/stable-diffusion-xl-base-1.0 unet: 1680 tensors, 2.57 B parameters
 
 
-def test_sdxl_vae_decoder_names_and_shapes():
-    d = ref_env.import_reference()
-    vae = _meta(d.AutoencoderKL, specs.SDXL_VAE_CONFIG)
-    _compare(specs.vae_decoder_params(specs.SDXL_VAE_CONFIG), vae, lambda k: k.startswith(("decoder.", "post_quant_conv.")))
+def test_sdxl_vae_decoder_names_and_shapes(reference_api):
+    _compare(specs.vae_decoder_params(specs.SDXL_VAE_CONFIG), reference_api["inventories"]["sdxl_vae"],
+             lambda k: k.startswith(("decoder.", "post_quant_conv.")))
 
 
-def test_flux_dev_names_and_shapes():
-    d = ref_env.import_reference()
-    _compare(specs.flux_params(specs.FLUX_DEV_CONFIG), _meta(d.FluxTransformer2DModel, specs.FLUX_DEV_CONFIG))
+def test_flux_dev_names_and_shapes(reference_api):
+    _compare(specs.flux_params(specs.FLUX_DEV_CONFIG), reference_api["inventories"]["flux_dev"])
 
 
-def test_ddpm_unet2d_names_and_shapes():
-    d = ref_env.import_reference()
-    _compare(specs.unet2d_params(specs.DDPM_TINY_CONFIG), _meta(d.UNet2DModel, specs.DDPM_TINY_CONFIG))
+def test_ddpm_unet2d_names_and_shapes(reference_api):
+    _compare(specs.unet2d_params(specs.DDPM_TINY_CONFIG), reference_api["inventories"]["ddpm_tiny"])
 
 
-def test_sdxl_vae_whole_checkpoint_names_and_shapes():
+def test_sdxl_vae_whole_checkpoint_names_and_shapes(reference_api):
     """encoder + quant_conv + post_quant_conv + decoder = the reference's whole AutoencoderKL state_dict (N3: encode)."""
-    d = ref_env.import_reference()
-    n = _compare(specs.vae_params(specs.SDXL_VAE_CONFIG), _meta(d.AutoencoderKL, specs.SDXL_VAE_CONFIG))
+    n = _compare(specs.vae_params(specs.SDXL_VAE_CONFIG), reference_api["inventories"]["sdxl_vae"])
     assert n == 248  # madebyollin/sdxl-vae-fp16-fix, stabilityai/sdxl-vae: 248 tensors
 
 
